@@ -18,6 +18,10 @@ Rank 0 prints ONE JSON line.
   cpu_baseline the CPU oracle (plain-C port of the algorithm, test infrastructure) on a bounded sample of the workload
   configs      driver-visible numbers for the other BASELINE configurations (cfg 3 and the horizon sweep at N=1 GPU;
                cfg 4 = 16 384 via-point instances split over the ranks of this run: strong scaling over the driver's runs)
+
+--dump-outputs DIR writes what the last timed step returned (on rank 0: instances [0, batch)) as DIR/<name>.npy, float64:
+u_seq [B, N, 2], x_seq [B, N, 3], dt, status, kkt_err, iters [B] and instance [B] (the instance index of each row).  Above
+64 MB in all, the rows are a fixed seeded sample.  The inputs are seeded, so two builds can be compared output for output.
 """
 import argparse
 import json
@@ -27,6 +31,7 @@ import sys
 import threading
 import time
 
+sys.dont_write_bytecode = True   # the benchmark writes nothing into the tree it runs from
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
 
@@ -149,10 +154,27 @@ class ClockSampler(threading.Thread):
                 "reasons": reasons, "samples": len(self.rows)}
 
 
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir, res):
+    """The arrays of one step's result dict as out_dir/<name>.npy (float64); rows sampled with a fixed seed above 64 MB."""
+    names = ("u_seq", "x_seq", "dt", "status", "kkt_err", "iters")
+    B = res["status"].shape[0]
+    row_bytes = 8 * (1 + sum(res[k][0].size for k in names))   # + the instance index
+    rows = np.arange(B)
+    budget = DUMP_LIMIT_BYTES - 4096   # room for the .npy headers
+    if B * row_bytes > budget:
+        rows = np.sort(np.random.default_rng(0).choice(B, budget // row_bytes, replace=False))
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "instance.npy"), rows.astype(np.float64))
+    for k in names:
+        np.save(os.path.join(out_dir, k + ".npy"), np.asarray(res[k][rows], dtype=np.float64))
+
+
 def cpu_arm(cfg, data_fn, seconds_target, threads):
     """The CPU oracle (port) on a bounded sample of the same workload, on the host threads this process may use."""
     from oracle import oracle_py as orc
-    orc.build()
     n = max(threads * 8, 32)
     data = data_fn(n)
     t = time.time()
@@ -180,6 +202,7 @@ def main():
     ap.add_argument("--batch", type=int, default=0, help="instances per GPU (default: the configuration's batch)")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-extra-configs", action="store_true", help="skip the secondary blocks (cfg 3 / 4 / horizon sweep / queue)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the results of the last timed step as DIR/<name>.npy")
     args = ap.parse_args()
     rank = int(os.environ.get("RANK", "0"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
@@ -199,7 +222,6 @@ def main():
         if rank != 0:
             return 0
         from oracle import oracle_py as orc
-        orc.build()
         sample = max(threads * 32, 256)
         data = configs.generate(cid, sample, n=n_h)
         for _ in range(max(args.warmup, 0)):
@@ -210,6 +232,8 @@ def main():
             out = orc.step_batch(cfg, data, n_threads=threads)
             conv += int((out["status"] == 0).sum())
         el = time.time() - t0
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs, out)
         val = conv / el
         print(json.dumps({
             "impl": "reference", "metric": metric, "value": val, "unit": UNIT, "n_gpus": args.gpus, "steps": args.steps,
@@ -312,7 +336,7 @@ def main():
         sampler.stop_flag = True
         st = solver.stats()
         res = solver.fetch()
-        out = {"el": el, "conv": int((res["status"] == 0).sum()), "iters_mean": float(res["iters"].mean()), "stats": st,
+        out = {"el": el, "res": res, "conv": int((res["status"] == 0).sum()), "iters_mean": float(res["iters"].mean()), "stats": st,
                "clocks": sampler.summary(), "solver": solver, "data": data, "timed": timed, "gather_controls": gather_controls}
         if want_e2e:
             keep = []
@@ -353,6 +377,8 @@ def main():
 
     # ================= the contract workload =================
     m = measure(cid, cfg, B, args.steps, args.warmup, rank * B, True, True)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, m["res"])
     (el, el_e2e), (conv_total, conv_e2e_total) = reduce_max_sum([m["el"], m["el_e2e"]], [m["conv"], m["conv_e2e"]])
     solver, st, N = m["solver"], m["stats"], cfg.n
 
