@@ -215,7 +215,8 @@ int mpcb200_step_batch(mpcb200_handle* h, int B, const double* x0, const double*
  * different instances are independent, so every instance gets exactly the result mpcb200_step_batch would give it from a
  * cold start; what changes is the cost: a batch pays max-over-instances iterations, the pool pays the mean.
  * Arrays as in mpcb200_step_batch with B = total; always a cold start, no x_init / reinit; outer_iterations must be 1.
- * Afterwards the handle is in the state after mpcb200_reset.
+ * The queue has device arrays of its own: the resident batch (its inputs, its warm state and its iteration history) is left
+ * as it was, and mpcb200_solve_resident / mpcb200_fetch_results afterwards see the batch of the last upload.
  */
 int mpcb200_solve_stream(mpcb200_handle* h, int total, const double* x0, const double* xf, const double* u_prev, double u_prev_dt,
                          const mpcb200_obstacles* obst, const mpcb200_viapoints* vp, double* u_seq, double* x_seq, double* dt_out,

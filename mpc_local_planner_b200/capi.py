@@ -181,6 +181,25 @@ def pack_viapoints(count, poses):
     return v, (count, poses)
 
 
+def pack_costmaps(cost, origin, resolution):
+    """cost [B, size_y, size_x] uint8, origin [B, 2] -> (Costmaps struct, keep-alive tuple (cost, origin))."""
+    cost = np.ascontiguousarray(cost, dtype=np.uint8)
+    origin = np.ascontiguousarray(origin, dtype=np.float64)
+    m = Costmaps(cost.shape[2], cost.shape[1], float(resolution), _dp(origin), cost.ctypes.data_as(C.POINTER(C.c_ubyte)))
+    return m, (cost, origin)
+
+
+def _results(B, N):
+    """host arrays for the results of B instances"""
+    return dict(u_seq=np.empty((B, N, 2)), x_seq=np.empty((B, N, 3)), dt=np.empty(B),
+                status=np.empty(B, dtype=np.int32), kkt_err=np.empty(B), iters=np.empty(B, dtype=np.int32))
+
+
+def _result_ptrs(out):
+    """the output arguments u_seq, x_seq, dt, status, kkt_err, iters of the C calls"""
+    return (_dp(out["u_seq"]), _dp(out["x_seq"]), _dp(out["dt"]), _ip(out["status"]), _dp(out["kkt_err"]), _ip(out["iters"]))
+
+
 _LIB = None
 _PKG_DIR = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.path.join(_PKG_DIR, "libmpcb200.so")
@@ -320,13 +339,11 @@ class BatchSolver:
     def solve_stream(self, x0, xf, u_prev=None, u_prev_dt=0.0, obstacles=None, viapoints=None):
         """A queue of len(x0) instances (any number) through the pool of max_batch slots: continuous batching, cold starts."""
         T, x0, xf, u_prev, o, v, xi, keep = self._prep_inputs(x0, xf, u_prev, obstacles, viapoints, None)
-        N = self.N
-        out = dict(u_seq=np.empty((T, N, 2)), x_seq=np.empty((T, N, 3)), dt=np.empty(T),
-                   status=np.empty(T, dtype=np.int32), kkt_err=np.empty(T), iters=np.empty(T, dtype=np.int32))
+        out = _results(T, self.N)
         t = C.c_double(0.0)
         rc = self.lib.mpcb200_solve_stream(
             self.h, T, _dp(x0), _dp(xf), _dp(u_prev), float(u_prev_dt), C.byref(o) if o else None, C.byref(v) if v else None,
-            _dp(out["u_seq"]), _dp(out["x_seq"]), _dp(out["dt"]), _ip(out["status"]), _dp(out["kkt_err"]), _ip(out["iters"]), C.byref(t))
+            *_result_ptrs(out), C.byref(t))
         self._check(rc, "mpcb200_solve_stream")
         out["solve_time_s"] = t.value
         return out
@@ -334,9 +351,7 @@ class BatchSolver:
     def alloc_outputs(self, B, pin=None):
         """Result buffers for step(..., out=...).  pin: optional callable array -> (pinned array, owner) (e.g. through
         torch.Tensor.pin_memory): page-locked buffers take the device-to-host copies without a staging copy."""
-        N = self.N
-        out = dict(u_seq=np.empty((B, N, 2)), x_seq=np.empty((B, N, 3)), dt=np.empty(B),
-                   status=np.empty(B, dtype=np.int32), kkt_err=np.empty(B), iters=np.empty(B, dtype=np.int32))
+        out = _results(B, self.N)
         if pin is not None:
             owners = []
             for k in list(out):
@@ -349,7 +364,6 @@ class BatchSolver:
         """Controller::step for a batch (host arrays in, host arrays out; copies inside the call).  out: buffers of
         alloc_outputs() to write the results into (default: fresh arrays)."""
         B, x0, xf, u_prev, o, v, xi, keep = self._prep_inputs(x0, xf, u_prev, obstacles, viapoints, x_init)
-        N = self.N
         if out is None:
             out = self.alloc_outputs(B)
         t = C.c_double(0.0)
@@ -359,8 +373,7 @@ class BatchSolver:
         rc = self.lib.mpcb200_step_batch(
             self.h, B, _dp(x0), _dp(xf), _dp(u_prev), float(u_prev_dt), C.byref(o) if o else None,
             C.byref(v) if v else None, _dp(xi), ri.ctypes.data_as(C.POINTER(C.c_ubyte)) if ri is not None else None,
-            _dp(out["u_seq"]), _dp(out["x_seq"]), _dp(out["dt"]), _ip(out["status"]), _dp(out["kkt_err"]),
-            _ip(out["iters"]), C.byref(t))
+            *_result_ptrs(out), C.byref(t))
         self._check(rc, "mpcb200_step_batch")
         out["solve_time_s"] = t.value
         self.B = B
@@ -379,12 +392,8 @@ class BatchSolver:
         return t.value
 
     def fetch(self):
-        B, N = self.B, self.N
-        out = dict(u_seq=np.empty((B, N, 2)), x_seq=np.empty((B, N, 3)), dt=np.empty(B),
-                   status=np.empty(B, dtype=np.int32), kkt_err=np.empty(B), iters=np.empty(B, dtype=np.int32))
-        rc = self.lib.mpcb200_fetch_results(self.h, _dp(out["u_seq"]), _dp(out["x_seq"]), _dp(out["dt"]),
-                                            _ip(out["status"]), _dp(out["kkt_err"]), _ip(out["iters"]))
-        self._check(rc, "mpcb200_fetch_results")
+        out = _results(self.B, self.N)
+        self._check(self.lib.mpcb200_fetch_results(self.h, *_result_ptrs(out)), "mpcb200_fetch_results")
         return out
 
     def reset(self, which=None):
@@ -397,10 +406,9 @@ class BatchSolver:
     def costmap_obstacles(self, cost, origin, resolution, robot_pose, behind_robot_dist, max_per_instance):
         """updateObstacleContainerWithCostmap for B robots: cost [B, size_y, size_x] uint8, origin [B, 2], robot_pose [B, 3]
         -> (count [B], type [B, M], params [B, M, OBST_STRIDE]) in the layout step() takes as `obstacles`, and found [B]."""
-        cost = np.ascontiguousarray(cost, dtype=np.uint8)
-        origin = np.ascontiguousarray(origin, dtype=np.float64); pose = np.ascontiguousarray(robot_pose, dtype=np.float64)
+        m, (cost, origin) = pack_costmaps(cost, origin, resolution)
+        pose = np.ascontiguousarray(robot_pose, dtype=np.float64)
         B, M = cost.shape[0], int(max_per_instance)
-        m = Costmaps(cost.shape[2], cost.shape[1], float(resolution), _dp(origin), cost.ctypes.data_as(C.POINTER(C.c_ubyte)))
         count = np.zeros(B, dtype=np.int32); found = np.zeros(B, dtype=np.int32)
         typ = np.zeros((B, M), dtype=np.int32); par = np.zeros((B, M, OBST_STRIDE))
         self._check(self.lib.mpcb200_costmap_obstacles(self.h, B, C.byref(m), _dp(pose), float(behind_robot_dist), M, _ip(count), _ip(found),
@@ -412,8 +420,7 @@ class BatchSolver:
         """One planning cycle from the costmaps (updateObstacleContainerWithCostmap with robot pose = x0, then Controller::step): the
         obstacle lists stay on the device.  Returns step()'s dict plus obst_found [B]."""
         B, x0, xf, u_prev, _, v, xi, keep = self._prep_inputs(x0, xf, u_prev, None, viapoints, x_init)
-        cost = np.ascontiguousarray(cost, dtype=np.uint8); origin = np.ascontiguousarray(origin, dtype=np.float64)
-        m = Costmaps(cost.shape[2], cost.shape[1], float(resolution), _dp(origin), cost.ctypes.data_as(C.POINTER(C.c_ubyte)))
+        m, maps_keep = pack_costmaps(cost, origin, resolution)
         if out is None:
             out = self.alloc_outputs(B)
         found = np.zeros(B, dtype=np.int32)
@@ -422,7 +429,7 @@ class BatchSolver:
         rc = self.lib.mpcb200_step_batch_costmap(
             self.h, B, _dp(x0), _dp(xf), _dp(u_prev), float(u_prev_dt), C.byref(m), float(behind_robot_dist), int(max_per_instance),
             C.byref(v) if v else None, _dp(xi), ri.ctypes.data_as(C.POINTER(C.c_ubyte)) if ri is not None else None,
-            _dp(out["u_seq"]), _dp(out["x_seq"]), _dp(out["dt"]), _ip(out["status"]), _dp(out["kkt_err"]), _ip(out["iters"]), _ip(found), C.byref(t))
+            *_result_ptrs(out), _ip(found), C.byref(t))
         self._check(rc, "mpcb200_step_batch_costmap")
         out["solve_time_s"] = t.value
         out["obst_found"] = found
@@ -433,10 +440,9 @@ class BatchSolver:
                        circumscribed_radius=0.0):
         """isPoseTrajectoryFeasible for B robots: cost [B, size_y, size_x] uint8, origin [B, 2], footprint [n_fp, 2] (robot frame);
         x_seq [B, n, 3] or None = the trajectories of the last solve on the device.  -> bool [B]"""
-        cost = np.ascontiguousarray(cost, dtype=np.uint8); origin = np.ascontiguousarray(origin, dtype=np.float64)
+        m, (cost, origin) = pack_costmaps(cost, origin, resolution)
         fp = np.ascontiguousarray(footprint, dtype=np.float64).reshape(-1, 2)
         B = cost.shape[0]
-        m = Costmaps(cost.shape[2], cost.shape[1], float(resolution), _dp(origin), cost.ctypes.data_as(C.POINTER(C.c_ubyte)))
         xs = np.ascontiguousarray(x_seq, dtype=np.float64) if x_seq is not None else None
         ok = np.zeros(B, dtype=np.uint8)
         self._check(self.lib.mpcb200_check_feasible(self.h, B, C.byref(m), _dp(xs), xs.shape[1] if xs is not None else 0, _dp(fp), fp.shape[0],
@@ -545,13 +551,11 @@ class MultiSolver:
 
     def step(self, x0, xf, u_prev=None, u_prev_dt=0.0, obstacles=None, viapoints=None):
         B, x0, xf, u_prev, o, v, xi, keep = BatchSolver._prep_inputs(x0, xf, u_prev, obstacles, viapoints, None)
-        N = self.N
-        out = dict(u_seq=np.empty((B, N, 2)), x_seq=np.empty((B, N, 3)), dt=np.empty(B),
-                   status=np.empty(B, dtype=np.int32), kkt_err=np.empty(B), iters=np.empty(B, dtype=np.int32))
+        out = _results(B, self.N)
         t = C.c_double(0.0)
         rc = self.lib.mpcb200_step_batch_multi(
             self.h, B, _dp(x0), _dp(xf), _dp(u_prev), float(u_prev_dt), C.byref(o) if o else None, C.byref(v) if v else None, None, None,
-            _dp(out["u_seq"]), _dp(out["x_seq"]), _dp(out["dt"]), _ip(out["status"]), _dp(out["kkt_err"]), _ip(out["iters"]), C.byref(t))
+            *_result_ptrs(out), C.byref(t))
         if rc != 0:
             raise SolverError(f"mpcb200_step_batch_multi failed ({rc}): {self.lib.mpcb200_multi_last_error(self.h).decode()}")
         out["solve_time_s"] = t.value

@@ -432,50 +432,85 @@ __global__ void flush_kernel(double* buf, size_t n)
 // =================================================================================================================
 // host side
 // =================================================================================================================
+// a CUDA resource that is released with its owner: device or pinned memory, an event, a stream
+template <class T, auto Release>
+struct Owned
+{
+    T v{};
+    Owned() = default;
+    Owned(const Owned&) = delete;
+    Owned& operator=(const Owned&) = delete;
+    ~Owned() { reset(); }
+    void reset() { if (v) Release(v); v = T{}; }
+    T* put() { reset(); return &v; }   // out-parameter of the call that creates the resource
+    operator T() const { return v; }
+};
+template <class T> using Dev = Owned<T*, cudaFree>;
+template <class T> static cudaError_t alloc(Dev<T>& buf, size_t count) { return cudaMalloc(buf.put(), count * sizeof(T)); }
+using Event = Owned<cudaEvent_t, cudaEventDestroy>;
+
+// compact inputs and outputs of `rows` instances on the device ([row][...] as in mpcb200.h), and what the last upload put there
+struct Job
+{
+    size_t rows = 0;   // instances the arrays hold
+    int m = 0;         // obstacles per instance the obstacle arrays hold
+    Dev<double> x0, xf, uprev, obst, vp, xinit;   // xinit: the resident batch only
+    Dev<int> obst_count, obst_type, vp_count;
+    Dev<unsigned char> reinit;                    // the resident batch only
+    Dev<double> useq, xseq, dt, kkt, upacked;
+    Dev<int> status, iters;
+    // the last upload
+    int B = 0;
+    double uprev_dt = 0.0;
+    int has_uprev = 0, has_xinit = 0, has_reinit = 0;
+    int obst_max = 0, vp_max = 0;   // list lengths per instance (0: no list)
+    int has_lines = 0;  // line obstacles, moving obstacles or midpoint differences: the kernels are launched with those (rarely used) paths compiled in
+
+    InputPtrs inputs() const
+    {
+        return InputPtrs{x0, xf, has_uprev ? uprev.v : nullptr, obst_max ? obst_count.v : nullptr, obst_type, obst, obst_max,
+                         vp_max ? vp_count.v : nullptr, vp, vp_max, has_xinit ? xinit.v : nullptr, has_reinit ? reinit.v : nullptr};
+    }
+    OutputPtrs outputs() const { return OutputPtrs{useq, xseq, dt, status, kkt, iters, upacked}; }
+};
+
 struct mpcb200_handle
 {
     Cfg cfg;
     WsLayout L;
-    int max_batch, device, B;
-    int n_cap;                  // horizon the buffers were sized for at create (mpcb200_resample moves cfg.n within [3, n_cap])
-    double* d_resample;         // scratch of mpcb200_resample, allocated on first use
-    void* d_cm; size_t cm_cap; double costmap_ms;
-    void* d_fz; size_t fz_cap;   // scratch of mpcb200_check_feasible (maps, trajectories, footprint, flags)  // scratch of mpcb200_costmap_obstacles (grown on demand), device ms of its last call
-    double* ws;
-    int num_sms, clock_khz;
-    int solve_mode;             // MPCB200_OPT_SOLVE_MODE: 0 fused persistent kernel (default), 1 one kernel per phase
-    unsigned timing_mask;       // phased mode: phases bracketed by CUDA events inside solve (bit = phase id)
-    cudaStream_t stream, own_stream;  // stream in use / the stream the handle created
-    // compact device input / output staging
-    double *d_x0, *d_xf, *d_uprev, *d_obst, *d_vp, *d_xinit;
-    int *d_obst_count, *d_obst_type, *d_vp_count;
-    unsigned char* d_reinit;
-    double *d_useq, *d_xseq, *d_dt, *d_kkt, *d_upacked;
-    int *d_status, *d_iters, *d_nactive, *d_queue;
-    unsigned long long* d_counters;
-    int* h_nactive;  // pinned, two poll slots
-    cudaEvent_t poll_ev[2], t0, t1, c0, c1;   // t: around a solve, c: around the costmap kernels
-    double* d_flush; size_t flush_n;
-    int has_obst, has_vp, has_xinit, has_reinit, obst_max, vp_max;
-    int d_obst_m, s_obst_m;   // obstacles per instance the staging arrays (batch / queue job) hold
-    // queue job (mpcb200_solve_stream): inputs / outputs of the whole queue on the device (grown on demand)
-    size_t stream_cap;
-    double *s_x0, *s_xf, *s_uprev, *s_obst, *s_vp, *s_useq, *s_xseq, *s_dt, *s_kkt, *s_upacked;
-    int *s_obst_count, *s_obst_type, *s_vp_count, *s_status, *s_iters;
-    int has_lines;  // line obstacles in the batch, moving obstacles or midpoint differences: the kernels are launched with those (rarely used) paths compiled in
-    double uprev_dt;
-    int fused_grid;  // CTAs of the last fused launch
-    int order_by_history; // MPCB200_OPT_ORDER_BY_HISTORY: batch queue longest-first by the previous solve's iteration counts
-    int hist_B;           // batch size of the last batch solve whose iteration counts are in d_iters (0: none)
-    int *d_prev_iters, *d_order;
-    int sm_phase_sync;    // MPCB200_OPT_SM_PHASE_SYNC: co-resident CTAs of the solve kernel enter the phases together
-    unsigned long long* d_smsync;
-    int max_ctas_per_sm;  // MPCB200_OPT_CTAS_PER_SM: cap on the resident CTAs per SM of the solve kernel (0 = what fits)
-    mpcb200_stats stats;
+    int max_batch = 0, device = 0;
+    int n_cap = 0;              // horizon the buffers were sized for at create (mpcb200_resample moves cfg.n within [3, n_cap])
+    int num_sms = 0, clock_khz = 0;
+    int solve_mode = 0;         // MPCB200_OPT_SOLVE_MODE: 0 fused persistent kernel (default), 1 one kernel per phase
+    unsigned timing_mask = 1u << MPCB200_PHASE_KKT;   // phased mode: phases bracketed by CUDA events inside solve (bit = phase id)
+    int order_by_history = 1;   // MPCB200_OPT_ORDER_BY_HISTORY: batch queue longest-first by the previous solve's iteration counts
+    int sm_phase_sync = -1;     // MPCB200_OPT_SM_PHASE_SYNC: co-resident CTAs of the solve kernel enter the phases together
+    int max_ctas_per_sm = 0;    // MPCB200_OPT_CTAS_PER_SM: cap on the resident CTAs per SM of the solve kernel (0 = what fits)
+    int fused_grid = 0;         // CTAs of the last fused launch
+    int hist_B = 0;             // batch size of the last batch solve whose iteration counts are in batch.iters (0: none)
+    Owned<cudaStream_t, cudaStreamDestroy> own_stream;   // the stream the handle created
+    cudaStream_t stream = nullptr;                       // the stream in use
+    Dev<double> ws;             // instance blocks [max_batch][L.stride]
+    Job batch;                  // the resident batch: its inputs and the results of its last solve
+    Job queue;                  // the last queue job (mpcb200_solve_stream), grown on demand
+    Dev<int> d_nactive, d_queue, d_prev_iters, d_order;
+    Dev<unsigned long long> d_counters, d_smsync;
+    Dev<double> d_flush;
+    size_t flush_n = (size_t)40 * 1024 * 1024;   // 320 MB > 126 MB L2
+    // scratch grown on demand: mpcb200_resample; the costmap kernels; mpcb200_check_feasible (maps, trajectories, footprint, flags)
+    Dev<double> d_resample; size_t resample_cap = 0;
+    Dev<char> d_cm; size_t cm_cap = 0;
+    Dev<char> d_fz; size_t fz_cap = 0;
+    double costmap_ms = 0.0;    // device ms of the last costmap call
+    Owned<int*, cudaFreeHost> h_nactive;   // two poll slots
+    Event poll_ev[2], t0, t1, c0, c1;      // t: around a solve, c: around the costmap kernels
+    mpcb200_stats stats{};
     std::vector<cudaEvent_t> ev;  // pool of event pairs
     std::vector<int> ev_phase;
-    size_t ev_used;
+    size_t ev_used = 0;
     std::string err;
+    // the members release their resources after this body, on the handle's device
+    ~mpcb200_handle() { cudaSetDevice(device); for (cudaEvent_t e : ev) cudaEventDestroy(e); }
 };
 
 static std::string g_create_err = "";
@@ -554,9 +589,80 @@ static int validate_config(const mpcb200_config* c, std::string& why)
 template <class K>
 static cudaError_t allow_smem(K kernel) { return cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, MAX_IMG_SMEM); }
 
+// grows a job to `rows` instances with room for `m` obstacles per instance; never shrinks, and what a grown array held is gone
+static int reserve(mpcb200_handle* h, Job& j, size_t rows, int m)
+{
+    if (rows <= j.rows && m <= j.m) return 0;
+    CK(cudaStreamSynchronize(h->stream));   // work in flight may still use the old arrays
+    if (rows > j.rows)
+    {
+        const size_t R = rows, N = (size_t)h->n_cap;   // sized for the largest horizon the handle can be resampled to
+        j.rows = 0;
+        CK(alloc(j.x0, R * 3)); CK(alloc(j.xf, R * 3)); CK(alloc(j.uprev, R * 2)); CK(alloc(j.obst_count, R));
+        CK(alloc(j.vp, R * MAX_VP * 3)); CK(alloc(j.vp_count, R));
+        CK(alloc(j.useq, R * N * 2)); CK(alloc(j.xseq, R * N * 3)); CK(alloc(j.dt, R)); CK(alloc(j.kkt, R));
+        CK(alloc(j.upacked, R * (N - 1) * 2)); CK(alloc(j.status, R)); CK(alloc(j.iters, R));
+        j.rows = rows;
+    }
+    const size_t M = (size_t)(m > j.m ? m : j.m);
+    j.m = 0;
+    CK(alloc(j.obst, j.rows * M * MPCB200_OBST_STRIDE)); CK(alloc(j.obst_type, j.rows * M));
+    j.m = (int)M;
+    return 0;
+}
+
+// obstacles per instance a job needs for `obst` (longer lists than the ABI accepts are refused by the upload)
+static int obstacle_room(const mpcb200_obstacles* obst)
+{
+    const int m = (obst && obst->count) ? obst->max_per_instance : 0;
+    return m > MAX_OBST && m <= MAX_OBST_LIST ? m : MAX_OBST;
+}
+
+// scratch that grows on demand; what it held is gone
+template <class T> static int grow(mpcb200_handle* h, Dev<T>& buf, size_t& cap, size_t bytes)
+{
+    if (bytes <= cap) return 0;
+    CK(cudaStreamSynchronize(h->stream));   // work in flight may still use the old buffer
+    cap = 0;
+    CK(cudaMalloc(buf.put(), bytes));
+    cap = bytes;
+    return 0;
+}
+
+// everything on the device a handle needs from the start
+static int init_device(mpcb200_handle* h)
+{
+    CK(cudaSetDevice(h->device));
+    CK(cudaStreamCreateWithFlags(h->own_stream.put(), cudaStreamNonBlocking));
+    h->stream = h->own_stream;
+    const size_t B = (size_t)h->max_batch;
+    int rc = reserve(h, h->batch, B, MAX_OBST);
+    if (rc) return rc;
+    CK(alloc(h->batch.xinit, B * h->n_cap * 3)); CK(alloc(h->batch.reinit, B));
+    CK(alloc(h->ws, B * h->L.stride));
+    CK(cudaMemsetAsync(h->ws, 0, B * h->L.stride * sizeof(double), h->stream));
+    CK(cudaDeviceGetAttribute(&h->num_sms, cudaDevAttrMultiProcessorCount, h->device));
+    CK(cudaDeviceGetAttribute(&h->clock_khz, cudaDevAttrClockRate, h->device));
+    CK(alloc(h->d_nactive, 2)); CK(alloc(h->d_queue, 1)); CK(alloc(h->d_smsync, 1024)); CK(alloc(h->d_prev_iters, B)); CK(alloc(h->d_order, B));
+    CK(alloc(h->d_counters, CNT_WORDS)); CK(cudaMemsetAsync(h->d_counters, 0, CNT_WORDS * 8, h->stream));
+    CK(allow_smem(phase_kernel<false>)); CK(allow_smem(phase_kernel<true>));
+    CK(allow_smem(kkt_warp_kernel<false>)); CK(allow_smem(kkt_warp_kernel<true>));
+    CK(allow_smem(solve_fused_kernel<false, false>)); CK(allow_smem(solve_fused_kernel<false, true>));
+    CK(allow_smem(solve_fused_kernel<true, false>)); CK(allow_smem(solve_fused_kernel<true, true>));
+    CK(cudaMallocHost(h->h_nactive.put(), 8));
+    CK(cudaEventCreateWithFlags(h->poll_ev[0].put(), cudaEventDisableTiming)); CK(cudaEventCreateWithFlags(h->poll_ev[1].put(), cudaEventDisableTiming));
+    CK(cudaEventCreate(h->t0.put())); CK(cudaEventCreate(h->t1.put())); CK(cudaEventCreate(h->c0.put())); CK(cudaEventCreate(h->c1.put()));
+    CK(alloc(h->d_flush, h->flush_n));
+    CK(cudaMemsetAsync(h->d_flush, 0, h->flush_n * 8, h->stream));
+    // all instances start cold
+    reset_kernel<<<(h->max_batch + 127) / 128, 128, 0, h->stream>>>(h->L, h->ws, h->max_batch, nullptr);
+    CK(cudaGetLastError());
+    CK(cudaStreamSynchronize(h->stream));
+    return 0;
+}
+
 extern "C" int mpcb200_create(const mpcb200_config* cfg, int max_batch, int device, mpcb200_handle** out)
 {
-    mpcb200_handle* h = nullptr;
     if (!cfg || !out || max_batch < 1) return set_err(nullptr, MPCB200_E_INVALID, "bad arguments");
     std::string why;
     int rc = validate_config(cfg, why);
@@ -566,55 +672,15 @@ extern "C" int mpcb200_create(const mpcb200_config* cfg, int max_batch, int devi
     if (e != cudaSuccess || ndev == 0)
         return set_err(nullptr, MPCB200_E_NODEVICE, std::string("no CUDA device (") + cudaGetErrorString(e) + "): this solver has no CPU fallback");
     if (device < 0 || device >= ndev) return set_err(nullptr, MPCB200_E_INVALID, "device index out of range");
-    h = new mpcb200_handle();
-    h->cfg = *cfg; h->max_batch = max_batch; h->device = device; h->B = 0; h->ws = nullptr; h->ev_used = 0;
-    memset(&h->stats, 0, sizeof(h->stats));
+    mpcb200_handle* h = new mpcb200_handle();
+    h->cfg = *cfg; h->max_batch = max_batch; h->device = device; h->n_cap = cfg->n;
     make_layout(cfg, MAX_OBST, MAX_VP, h->L);
-    h->n_cap = cfg->n; h->d_resample = nullptr; h->d_cm = nullptr; h->cm_cap = 0; h->costmap_ms = 0.0; h->d_fz = nullptr; h->fz_cap = 0;
-    h->uprev_dt = 0.0; h->has_obst = h->has_vp = h->has_xinit = h->has_reinit = 0; h->obst_max = h->vp_max = 0; h->has_lines = 0;
-    h->solve_mode = 0; h->timing_mask = 1u << MPCB200_PHASE_KKT; h->fused_grid = 0; h->max_ctas_per_sm = 0; h->sm_phase_sync = -1; h->d_smsync = nullptr; h->order_by_history = 1; h->hist_B = 0; h->d_prev_iters = h->d_order = nullptr;
-#define CKC(call)                                                                                                  \
-    do {                                                                                                           \
-        cudaError_t e_ = (call);                                                                                   \
-        if (e_ != cudaSuccess) { std::string m = std::string(#call) + ": " + cudaGetErrorString(e_); delete h; return set_err(nullptr, MPCB200_E_CUDA, m); } \
-    } while (0)
-    CKC(cudaSetDevice(device));
-    CKC(cudaStreamCreateWithFlags(&h->own_stream, cudaStreamNonBlocking));
-    h->stream = h->own_stream;
-    const size_t B = (size_t)max_batch, N = (size_t)cfg->n;
-    CKC(cudaMalloc(&h->ws, B * h->L.stride * sizeof(double)));
-    CKC(cudaMemsetAsync(h->ws, 0, B * h->L.stride * sizeof(double), h->stream));
-    CKC(cudaDeviceGetAttribute(&h->num_sms, cudaDevAttrMultiProcessorCount, device));
-    CKC(cudaDeviceGetAttribute(&h->clock_khz, cudaDevAttrClockRate, device));
-    CKC(cudaMalloc(&h->d_x0, B * 3 * 8)); CKC(cudaMalloc(&h->d_xf, B * 3 * 8)); CKC(cudaMalloc(&h->d_uprev, B * 2 * 8));
-    CKC(cudaMalloc(&h->d_obst, B * MAX_OBST * MPCB200_OBST_STRIDE * 8)); CKC(cudaMalloc(&h->d_obst_count, B * 4));
-    CKC(cudaMalloc(&h->d_obst_type, B * MAX_OBST * 4));
-    h->d_obst_m = MAX_OBST; h->s_obst_m = 0;
-    CKC(cudaMalloc(&h->d_vp, B * MAX_VP * 3 * 8)); CKC(cudaMalloc(&h->d_vp_count, B * 4));
-    CKC(cudaMalloc(&h->d_xinit, B * N * 3 * 8)); CKC(cudaMalloc(&h->d_reinit, B));
-    CKC(cudaMalloc(&h->d_useq, B * N * 2 * 8)); CKC(cudaMalloc(&h->d_xseq, B * N * 3 * 8)); CKC(cudaMalloc(&h->d_dt, B * 8));
-    CKC(cudaMalloc(&h->d_kkt, B * 8)); CKC(cudaMalloc(&h->d_upacked, B * (N - 1) * 2 * 8));
-    CKC(cudaMalloc(&h->d_status, B * 4)); CKC(cudaMalloc(&h->d_iters, B * 4)); CKC(cudaMalloc(&h->d_nactive, 8)); CKC(cudaMalloc(&h->d_queue, 4)); CKC(cudaMalloc(&h->d_smsync, 1024 * 8)); CKC(cudaMalloc(&h->d_prev_iters, B * 4)); CKC(cudaMalloc(&h->d_order, B * 4));
-    CKC(cudaMalloc(&h->d_counters, CNT_WORDS * 8)); CKC(cudaMemsetAsync(h->d_counters, 0, CNT_WORDS * 8, h->stream));
-    CKC(allow_smem(phase_kernel<false>)); CKC(allow_smem(phase_kernel<true>));
-    CKC(allow_smem(kkt_warp_kernel<false>)); CKC(allow_smem(kkt_warp_kernel<true>));
-    CKC(allow_smem(solve_fused_kernel<false, false>)); CKC(allow_smem(solve_fused_kernel<false, true>));
-    CKC(allow_smem(solve_fused_kernel<true, false>)); CKC(allow_smem(solve_fused_kernel<true, true>));
-    CKC(cudaMallocHost(&h->h_nactive, 8));
-    h->stream_cap = 0;
-    h->s_x0 = h->s_xf = h->s_uprev = h->s_obst = h->s_vp = h->s_useq = h->s_xseq = h->s_dt = h->s_kkt = h->s_upacked = nullptr;
-    h->s_obst_count = h->s_obst_type = h->s_vp_count = h->s_status = h->s_iters = nullptr;
-    CKC(cudaEventCreateWithFlags(&h->poll_ev[0], cudaEventDisableTiming)); CKC(cudaEventCreateWithFlags(&h->poll_ev[1], cudaEventDisableTiming));
-    CKC(cudaEventCreate(&h->t0)); CKC(cudaEventCreate(&h->t1)); CKC(cudaEventCreate(&h->c0)); CKC(cudaEventCreate(&h->c1));
-    h->flush_n = (size_t)40 * 1024 * 1024;  // 320 MB > 126 MB L2
-    CKC(cudaMalloc(&h->d_flush, h->flush_n * 8));
-    CKC(cudaMemsetAsync(h->d_flush, 0, h->flush_n * 8, h->stream));
+    if ((rc = init_device(h)))
     {
-        // all instances start cold
-        reset_kernel<<<(max_batch + 127) / 128, 128, 0, h->stream>>>(h->L, h->ws, max_batch, nullptr);
-        CKC(cudaGetLastError());
+        why = h->err;
+        delete h;
+        return set_err(nullptr, rc, why);
     }
-    CKC(cudaStreamSynchronize(h->stream));
     *out = h;
     return MPCB200_OK;
 }
@@ -624,16 +690,6 @@ extern "C" void mpcb200_destroy(mpcb200_handle* h)
     if (!h) return;
     cudaSetDevice(h->device);
     cudaStreamSynchronize(h->stream);
-    void* ptrs[] = {h->ws, h->d_x0, h->d_xf, h->d_uprev, h->d_obst, h->d_obst_count, h->d_obst_type, h->d_vp, h->d_vp_count, h->d_xinit,
-                    h->d_reinit, h->d_useq, h->d_xseq, h->d_dt, h->d_kkt, h->d_upacked, h->d_status, h->d_iters, h->d_nactive, h->d_queue, h->d_flush, h->d_counters, h->d_smsync, h->d_prev_iters, h->d_order};
-    for (void* p : ptrs) if (p) cudaFree(p);
-    void* sptrs[] = {h->s_x0, h->s_xf, h->s_uprev, h->s_obst, h->s_vp, h->s_useq, h->s_xseq, h->s_dt, h->s_kkt, h->s_upacked, h->s_obst_count,
-                     h->s_obst_type, h->s_vp_count, h->s_status, h->s_iters, h->d_resample, h->d_cm, h->d_fz};
-    for (void* p : sptrs) if (p) cudaFree(p);
-    if (h->h_nactive) cudaFreeHost(h->h_nactive);
-    for (auto& e : h->ev) cudaEventDestroy(e);
-    cudaEventDestroy(h->poll_ev[0]); cudaEventDestroy(h->poll_ev[1]); cudaEventDestroy(h->t0); cudaEventDestroy(h->t1); cudaEventDestroy(h->c0); cudaEventDestroy(h->c1);
-    cudaStreamDestroy(h->own_stream);
     delete h;
 }
 
@@ -678,12 +734,12 @@ static int group_threads(const mpcb200_handle* h)
     const int gw = (h->cfg.n + 31) / 32;
     return 32 * (gw < MAX_GROUP_WARPS ? gw : MAX_GROUP_WARPS);   // a lane per stage
 }
-static int image_words(const mpcb200_handle* h) { return resident_words(h->L, h->has_obst ? (h->obst_max < h->L.M ? h->obst_max : h->L.M) : 0); }
+static int image_words(const mpcb200_handle* h, const Job& j) { return resident_words(h->L, j.obst_max < h->L.M ? j.obst_max : h->L.M); }
 
-static InputPtrs batch_inputs(mpcb200_handle* h, bool with_uprev);
 static int launch_phase(mpcb200_handle* h, int phase, int B, int force_cold, int first_outer, int* n_active, bool timed)
 {
-    const int img_words = image_words(h);
+    const Job& j = h->batch;
+    const int img_words = image_words(h, j);
     const size_t img_smem = IMG_HEAD + (size_t)img_words * 8;
     if (img_smem > MAX_IMG_SMEM) return set_err(h, MPCB200_E_UNSUPPORTED, "the instance does not fit in shared memory");
     if (timed && ev_begin(h, phase)) return set_err(h, MPCB200_E_CUDA, "cudaEventCreate failed");
@@ -694,8 +750,8 @@ static int launch_phase(mpcb200_handle* h, int phase, int B, int force_cold, int
     }
     else if (phase >= 0 && phase < MPCB200_NUM_PHASES)
     {
-        if (h->has_lines) phase_kernel<true><<<B, group_threads(h), img_smem, h->stream>>>(h->cfg, h->L, h->ws, B, phase, h->uprev_dt, force_cold, first_outer, n_active, img_words, batch_inputs(h, true));
-        else phase_kernel<false><<<B, group_threads(h), img_smem, h->stream>>>(h->cfg, h->L, h->ws, B, phase, h->uprev_dt, force_cold, first_outer, n_active, img_words, batch_inputs(h, true));
+        const auto kernel = j.has_lines ? phase_kernel<true> : phase_kernel<false>;
+        kernel<<<B, group_threads(h), img_smem, h->stream>>>(h->cfg, h->L, h->ws, B, phase, j.uprev_dt, force_cold, first_outer, n_active, img_words, j.inputs());
     }
     else return set_err(h, MPCB200_E_INVALID, "unknown phase");
     if (timed) ev_end(h);
@@ -711,127 +767,88 @@ static int check_batch(mpcb200_handle* h, int B)
     return 0;
 }
 
-// which kernel variants a batch needs: line obstacles among the obstacles in use (padding slots are never read)
-static int scan_obstacles(mpcb200_handle* h, size_t B, const mpcb200_obstacles* obst)
+// which kernel variants a job needs: line obstacles among the obstacles in use (padding slots are never read)
+static bool has_line_obstacles(size_t B, const mpcb200_obstacles* obst)
 {
     const size_t M = (size_t)obst->max_per_instance;
-    int lines = 0;
     for (size_t b = 0; b < B; ++b)
     {
         const int cnt = obst->count[b] < (int)M ? obst->count[b] : (int)M;
-        for (int i = 0; i < cnt; ++i) lines |= obst->type[b * M + i] == MPCB200_OBST_LINE;
+        for (int i = 0; i < cnt; ++i)
+            if (obst->type[b * M + i] == MPCB200_OBST_LINE) return true;
     }
-    h->has_lines = lines || h->cfg.enable_dynamic_obstacles || is_midpoint(h->cfg);
-    return 0;
+    return false;
 }
 
-// host -> device copies of the inputs of `B` instances into the compact staging arrays d (batch) or s (queue job)
-struct Staging { double *x0, *xf, *uprev, *obst, *vp, *xinit; int *obst_count, *obst_type, *vp_count; unsigned char* reinit; };
-static int copy_inputs(mpcb200_handle* h, const Staging& d, size_t B, const double* x0, const double* xf, const double* u_prev, double u_prev_dt,
-                       const mpcb200_obstacles* obst, const mpcb200_viapoints* vp, const double* x_init, const unsigned char* reinit, InputPtrs* in)
+// host -> device copies of the inputs of `B` instances into a job (grown to hold them), and their description
+static int upload(mpcb200_handle* h, Job& j, size_t B, const double* x0, const double* xf, const double* u_prev, double u_prev_dt,
+                  const mpcb200_obstacles* obst, const mpcb200_viapoints* vp, const double* x_init, const unsigned char* reinit)
 {
     if (!x0 || !xf) return set_err(h, MPCB200_E_INVALID, "x0 and xf are required");
+    int rc = reserve(h, j, B, obstacle_room(obst));
+    if (rc) return rc;
     const size_t N = (size_t)h->cfg.n;
-    CK(cudaMemcpyAsync(d.x0, x0, B * 3 * 8, cudaMemcpyHostToDevice, h->stream));
-    CK(cudaMemcpyAsync(d.xf, xf, B * 3 * 8, cudaMemcpyHostToDevice, h->stream));
+    CK(cudaMemcpyAsync(j.x0, x0, B * 3 * 8, cudaMemcpyHostToDevice, h->stream));
+    CK(cudaMemcpyAsync(j.xf, xf, B * 3 * 8, cudaMemcpyHostToDevice, h->stream));
     h->stats.h2d_bytes += (long long)(B * 6 * 8);
-    if (u_prev) { CK(cudaMemcpyAsync(d.uprev, u_prev, B * 2 * 8, cudaMemcpyHostToDevice, h->stream)); h->stats.h2d_bytes += (long long)(B * 16); }
-    h->uprev_dt = u_prev_dt;
-    h->has_obst = 0; h->obst_max = 0; h->has_lines = is_midpoint(h->cfg);  // the kernel variants with the rarely used paths compiled in
+    j.has_uprev = u_prev != nullptr;
+    if (u_prev) { CK(cudaMemcpyAsync(j.uprev, u_prev, B * 2 * 8, cudaMemcpyHostToDevice, h->stream)); h->stats.h2d_bytes += (long long)(B * 16); }
+    j.uprev_dt = u_prev_dt;
+    j.obst_max = 0; j.has_lines = is_midpoint(h->cfg);
     if (obst && obst->count && obst->max_per_instance > 0)
     {
         if (obst->max_per_instance > MAX_OBST_LIST) return set_err(h, MPCB200_E_UNSUPPORTED, "more than 2048 obstacles per instance");
         if (!obst->type || !obst->params) return set_err(h, MPCB200_E_INVALID, "obstacle types and parameters are required");
         const size_t M = (size_t)obst->max_per_instance;
-        scan_obstacles(h, B, obst);
-        CK(cudaMemcpyAsync(d.obst_count, obst->count, B * 4, cudaMemcpyHostToDevice, h->stream));
-        CK(cudaMemcpyAsync(d.obst_type, obst->type, B * M * 4, cudaMemcpyHostToDevice, h->stream));
-        CK(cudaMemcpyAsync(d.obst, obst->params, B * M * MPCB200_OBST_STRIDE * 8, cudaMemcpyHostToDevice, h->stream));
+        j.has_lines = has_line_obstacles(B, obst) || h->cfg.enable_dynamic_obstacles || is_midpoint(h->cfg);
+        CK(cudaMemcpyAsync(j.obst_count, obst->count, B * 4, cudaMemcpyHostToDevice, h->stream));
+        CK(cudaMemcpyAsync(j.obst_type, obst->type, B * M * 4, cudaMemcpyHostToDevice, h->stream));
+        CK(cudaMemcpyAsync(j.obst, obst->params, B * M * MPCB200_OBST_STRIDE * 8, cudaMemcpyHostToDevice, h->stream));
         h->stats.h2d_bytes += (long long)(B * 4 + B * M * 4 + B * M * MPCB200_OBST_STRIDE * 8);
-        h->has_obst = 1; h->obst_max = (int)M;
+        j.obst_max = (int)M;
     }
-    h->has_vp = 0; h->vp_max = 0;
+    j.vp_max = 0;
     if (vp && vp->count && vp->max_per_instance > 0)
     {
         if (vp->max_per_instance > MAX_VP) return set_err(h, MPCB200_E_UNSUPPORTED, "more than 8 via-points per instance");
         const size_t V = (size_t)vp->max_per_instance;
-        CK(cudaMemcpyAsync(d.vp_count, vp->count, B * 4, cudaMemcpyHostToDevice, h->stream));
-        CK(cudaMemcpyAsync(d.vp, vp->poses, B * V * 3 * 8, cudaMemcpyHostToDevice, h->stream));
+        CK(cudaMemcpyAsync(j.vp_count, vp->count, B * 4, cudaMemcpyHostToDevice, h->stream));
+        CK(cudaMemcpyAsync(j.vp, vp->poses, B * V * 3 * 8, cudaMemcpyHostToDevice, h->stream));
         h->stats.h2d_bytes += (long long)(B * 4 + B * V * 24);
-        h->has_vp = 1; h->vp_max = (int)V;
+        j.vp_max = (int)V;
     }
-    h->has_xinit = 0;
-    if (x_init && d.xinit) { CK(cudaMemcpyAsync(d.xinit, x_init, B * N * 3 * 8, cudaMemcpyHostToDevice, h->stream)); h->has_xinit = 1; h->stats.h2d_bytes += (long long)(B * N * 24); }
-    h->has_reinit = 0;
-    if (reinit && d.reinit) { CK(cudaMemcpyAsync(d.reinit, reinit, B, cudaMemcpyHostToDevice, h->stream)); h->has_reinit = 1; h->stats.h2d_bytes += (long long)B; }
-    in->x0 = d.x0; in->xf = d.xf; in->u_prev = u_prev ? d.uprev : nullptr;
-    in->obst_count = h->has_obst ? d.obst_count : nullptr; in->obst_type = d.obst_type; in->obst_params = d.obst; in->obst_max = h->obst_max;
-    in->vp_count = h->has_vp ? d.vp_count : nullptr; in->vp_poses = d.vp; in->vp_max = h->vp_max;
-    in->x_init = h->has_xinit ? d.xinit : nullptr;
-    in->reinit = h->has_reinit ? d.reinit : nullptr;
+    j.has_xinit = x_init != nullptr;
+    if (x_init) { CK(cudaMemcpyAsync(j.xinit, x_init, B * N * 3 * 8, cudaMemcpyHostToDevice, h->stream)); h->stats.h2d_bytes += (long long)(B * N * 24); }
+    j.has_reinit = reinit != nullptr;
+    if (reinit) { CK(cudaMemcpyAsync(j.reinit, reinit, B, cudaMemcpyHostToDevice, h->stream)); h->stats.h2d_bytes += (long long)B; }
+    j.B = (int)B;
     return 0;
-}
-// obstacle lists longer than the resident list: the staging arrays grow to the list length on first use
-static int reserve_obstacles(mpcb200_handle* h, bool queue, size_t rows, int max_per_instance)
-{
-    if (max_per_instance <= 0 || max_per_instance > MAX_OBST_LIST) return 0;
-    int& cap = queue ? h->s_obst_m : h->d_obst_m;
-    if (max_per_instance <= cap) return 0;
-    double*& par = queue ? h->s_obst : h->d_obst;
-    int*& typ = queue ? h->s_obst_type : h->d_obst_type;
-    CK(cudaStreamSynchronize(h->stream));
-    if (par) cudaFree(par);
-    if (typ) cudaFree(typ);
-    par = nullptr; typ = nullptr; cap = 0;
-    const size_t M = (size_t)max_per_instance;
-    CK(cudaMalloc(&par, rows * M * MPCB200_OBST_STRIDE * 8));
-    CK(cudaMalloc(&typ, rows * M * 4));
-    cap = (int)M;
-    return 0;
-}
-static Staging batch_staging(mpcb200_handle* h) { return Staging{h->d_x0, h->d_xf, h->d_uprev, h->d_obst, h->d_vp, h->d_xinit, h->d_obst_count, h->d_obst_type, h->d_vp_count, h->d_reinit}; }
-static InputPtrs batch_inputs(mpcb200_handle* h, bool with_uprev)
-{
-    InputPtrs in;
-    in.x0 = h->d_x0; in.xf = h->d_xf; in.u_prev = with_uprev ? h->d_uprev : nullptr;
-    in.obst_count = h->has_obst ? h->d_obst_count : nullptr; in.obst_type = h->d_obst_type; in.obst_params = h->d_obst; in.obst_max = h->obst_max;
-    in.vp_count = h->has_vp ? h->d_vp_count : nullptr; in.vp_poses = h->d_vp; in.vp_max = h->vp_max;
-    in.x_init = h->has_xinit ? h->d_xinit : nullptr;
-    in.reinit = h->has_reinit ? h->d_reinit : nullptr;
-    return in;
 }
 
-static int upload_inputs(mpcb200_handle* h, int B, const double* x0, const double* xf, const double* u_prev, double u_prev_dt,
-                         const mpcb200_obstacles* obst, const mpcb200_viapoints* vp, const double* x_init, const unsigned char* reinit)
+// the resident batch's inputs into the instance blocks: the kernel-level API (phase kernels) works on the blocks
+static int scatter_batch(mpcb200_handle* h)
 {
-    CK(cudaSetDevice(h->device));
-    InputPtrs in;
-    if (!u_prev) CK(cudaMemsetAsync(h->d_uprev, 0, (size_t)B * 2 * 8, h->stream));
-    int rc = reserve_obstacles(h, false, (size_t)h->max_batch, (obst && obst->count) ? obst->max_per_instance : 0);
-    if (rc) return rc;
-    rc = copy_inputs(h, batch_staging(h), (size_t)B, x0, xf, u_prev, u_prev_dt, obst, vp, x_init, reinit, &in);
-    if (rc) return rc;
-    // the instance blocks get the inputs as well: the kernel-level API (phase kernels) works on the blocks
-    in.u_prev = h->d_uprev;
-    scatter_inputs_kernel<<<grid_for(B, WARPS_PER_CTA), WARPS_PER_CTA * 32, 0, h->stream>>>(h->L, h->ws, B, in);
+    const int B = h->batch.B;
+    scatter_inputs_kernel<<<grid_for(B, WARPS_PER_CTA), WARPS_PER_CTA * 32, 0, h->stream>>>(h->L, h->ws, B, h->batch.inputs());
     h->stats.launches_total += 1;
     CK(cudaGetLastError());
-    h->B = B;
     return 0;
 }
 
-// ---- the solve: one launch of the persistent kernel over a queue of `total` instances ----
-static int launch_fused(mpcb200_handle* h, int total, int queue_mode, int force_cold, const InputPtrs& in, const OutputPtrs& out)
+// ---- the solve: one launch of the persistent kernel over the instances of a job ----
+static int launch_fused(mpcb200_handle* h, const Job& j, int force_cold)
 {
+    const bool queue_mode = &j == &h->queue;   // cold instances without blocks (mpcb200_solve_stream)
+    const int total = j.B;
     FusedArgs a;
-    a.ws = h->ws; a.in = in; a.out = out; a.total = total; a.queue_mode = queue_mode; a.force_cold = force_cold; a.uprev_dt = h->uprev_dt;
-    a.img_words = image_words(h); a.queue = h->d_queue; a.counters = h->d_counters;
+    a.ws = h->ws; a.in = j.inputs(); a.out = j.outputs(); a.total = total; a.queue_mode = queue_mode; a.force_cold = force_cold; a.uprev_dt = j.uprev_dt;
+    a.img_words = image_words(h, j); a.queue = h->d_queue; a.counters = h->d_counters;
     a.sm_sync = nullptr; a.sm_gates = h->sm_phase_sync == 2 ? 2 : 3;
     a.order = nullptr;
     if (!queue_mode && h->order_by_history && h->hist_B == total && total > h->num_sms)
     {
-        // (d_iters is rewritten by this solve: order from a copy)
-        CK(cudaMemcpyAsync(h->d_prev_iters, h->d_iters, (size_t)total * 4, cudaMemcpyDeviceToDevice, h->stream));
+        // (the iteration counts are rewritten by this solve: order from a copy)
+        CK(cudaMemcpyAsync(h->d_prev_iters, j.iters, (size_t)total * 4, cudaMemcpyDeviceToDevice, h->stream));
         order_by_history_kernel<<<1, 1024, 0, h->stream>>>(h->d_prev_iters, total, h->d_order);
         h->stats.launches_total += 1;
         a.order = h->d_order;
@@ -841,26 +858,22 @@ static int launch_fused(mpcb200_handle* h, int total, int queue_mode, int force_
     if (smem > MAX_IMG_SMEM) return set_err(h, MPCB200_E_UNSUPPORTED, "the instance does not fit in shared memory");
     const int threads = group_threads(h);
     const bool ext = kkt_is_ext(h->cfg);
+    const auto kernel = j.has_lines ? (ext ? solve_fused_kernel<true, true> : solve_fused_kernel<true, false>)
+                                    : (ext ? solve_fused_kernel<false, true> : solve_fused_kernel<false, false>);
     int per_sm = 0;
-#define FUSED_DO(LN, EX)                                                                                                       \
-    do {                                                                                                                       \
-        CK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, solve_fused_kernel<LN, EX>, threads, smem));                 \
-        if (per_sm < 1) return set_err(h, MPCB200_E_UNSUPPORTED, "the solve kernel does not fit on an SM with this configuration"); \
-        if (h->max_ctas_per_sm > 0 && per_sm > h->max_ctas_per_sm) per_sm = h->max_ctas_per_sm;                                \
-        const int grid = total < per_sm * h->num_sms ? total : per_sm * h->num_sms;                                            \
-        h->fused_grid = grid;                                                                                                  \
-        /* phase alignment pays when several CTAs share an SM (auto: from three; measured, profiles/r2_phase_alignment.txt) */  \
-        if (h->sm_phase_sync > 0 || (h->sm_phase_sync < 0 && per_sm >= 3 && grid > h->num_sms))                                \
-        {                                                                                                                      \
-            a.sm_sync = h->d_smsync;                                                                                           \
-            CK(cudaMemsetAsync(h->d_smsync, 0, 1024 * 8, h->stream));                                                          \
-        }                                                                                                                      \
-        CK(cudaMemsetAsync(h->d_queue, 0, 4, h->stream));                                                                      \
-        solve_fused_kernel<LN, EX><<<grid, threads, smem, h->stream>>>(h->cfg, h->L, a);                                       \
-    } while (0)
-    if (h->has_lines) { if (ext) FUSED_DO(true, true); else FUSED_DO(true, false); }
-    else { if (ext) FUSED_DO(false, true); else FUSED_DO(false, false); }
-#undef FUSED_DO
+    CK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kernel, threads, smem));
+    if (per_sm < 1) return set_err(h, MPCB200_E_UNSUPPORTED, "the solve kernel does not fit on an SM with this configuration");
+    if (h->max_ctas_per_sm > 0 && per_sm > h->max_ctas_per_sm) per_sm = h->max_ctas_per_sm;
+    const int grid = total < per_sm * h->num_sms ? total : per_sm * h->num_sms;
+    h->fused_grid = grid;
+    // phase alignment pays when several CTAs share an SM (auto: from three; measured, profiles/r2_phase_alignment.txt)
+    if (h->sm_phase_sync > 0 || (h->sm_phase_sync < 0 && per_sm >= 3 && grid > h->num_sms))
+    {
+        a.sm_sync = h->d_smsync;
+        CK(cudaMemsetAsync(h->d_smsync, 0, 1024 * 8, h->stream));
+    }
+    CK(cudaMemsetAsync(h->d_queue, 0, 4, h->stream));
+    kernel<<<grid, threads, smem, h->stream>>>(h->cfg, h->L, a);
     h->stats.launches_total += 1;
     CK(cudaGetLastError());
     return 0;
@@ -904,8 +917,7 @@ static int solve_phased(mpcb200_handle* h, int B, int force_cold)
             if ((rc = launch_phase(h, MPCB200_PHASE_LINESEARCH, B, 0, 0, nullptr, timed(MPCB200_PHASE_LINESEARCH)))) return rc;
         }
     }
-    OutputPtrs o{h->d_useq, h->d_xseq, h->d_dt, h->d_status, h->d_kkt, h->d_iters, h->d_upacked};
-    gather_outputs_kernel<<<grid_for(B, WARPS_PER_CTA), WARPS_PER_CTA * 32, 0, h->stream>>>(h->L, h->ws, B, o);
+    gather_outputs_kernel<<<grid_for(B, WARPS_PER_CTA), WARPS_PER_CTA * 32, 0, h->stream>>>(h->L, h->ws, B, h->batch.outputs());
     h->stats.launches_total += 1;
     CK(cudaGetLastError());
     return 0;
@@ -926,16 +938,11 @@ static int collect_fused_counters(mpcb200_handle* h)
     return 0;
 }
 
-static int solve_device(mpcb200_handle* h, int B, int force_cold, double* solve_time_s)
+// the solve of a job (the resident batch: fused or phased; a queue: fused), timed with events, then the device counters
+static int solve_device(mpcb200_handle* h, const Job& j, int force_cold, double* solve_time_s)
 {
     CK(cudaEventRecord(h->t0, h->stream));
-    int rc;
-    if (h->solve_mode == 1) rc = solve_phased(h, B, force_cold);
-    else
-    {
-        OutputPtrs o{h->d_useq, h->d_xseq, h->d_dt, h->d_status, h->d_kkt, h->d_iters, h->d_upacked};
-        rc = launch_fused(h, B, 0, force_cold, batch_inputs(h, true), o);
-    }
+    const int rc = (&j == &h->batch && h->solve_mode == 1) ? solve_phased(h, j.B, force_cold) : launch_fused(h, j, force_cold);
     if (rc) return rc;
     CK(cudaEventRecord(h->t1, h->stream));
     CK(cudaStreamSynchronize(h->stream));
@@ -946,38 +953,21 @@ static int solve_device(mpcb200_handle* h, int B, int force_cold, double* solve_
     return collect_fused_counters(h);
 }
 
-static int fetch_results(mpcb200_handle* h, int B, double* u_seq, double* x_seq, double* dt_out, int* status, double* kkt_err, int* iters)
+// device -> host copies of the results of a job's last solve
+static int fetch(mpcb200_handle* h, const Job& j, double* u_seq, double* x_seq, double* dt_out, int* status, double* kkt_err, int* iters)
 {
-    const size_t N = (size_t)h->cfg.n;
-    if (u_seq) { CK(cudaMemcpyAsync(u_seq, h->d_useq, (size_t)B * N * 16, cudaMemcpyDeviceToHost, h->stream)); h->stats.d2h_bytes += (long long)(B * N * 16); }
-    if (x_seq) { CK(cudaMemcpyAsync(x_seq, h->d_xseq, (size_t)B * N * 24, cudaMemcpyDeviceToHost, h->stream)); h->stats.d2h_bytes += (long long)(B * N * 24); }
-    if (dt_out) { CK(cudaMemcpyAsync(dt_out, h->d_dt, (size_t)B * 8, cudaMemcpyDeviceToHost, h->stream)); h->stats.d2h_bytes += B * 8; }
-    if (status) { CK(cudaMemcpyAsync(status, h->d_status, (size_t)B * 4, cudaMemcpyDeviceToHost, h->stream)); h->stats.d2h_bytes += B * 4; }
-    if (kkt_err) { CK(cudaMemcpyAsync(kkt_err, h->d_kkt, (size_t)B * 8, cudaMemcpyDeviceToHost, h->stream)); h->stats.d2h_bytes += B * 8; }
-    if (iters) { CK(cudaMemcpyAsync(iters, h->d_iters, (size_t)B * 4, cudaMemcpyDeviceToHost, h->stream)); h->stats.d2h_bytes += B * 4; }
+    const size_t B = (size_t)j.B, N = (size_t)h->cfg.n;
+    if (u_seq) { CK(cudaMemcpyAsync(u_seq, j.useq, B * N * 16, cudaMemcpyDeviceToHost, h->stream)); h->stats.d2h_bytes += (long long)(B * N * 16); }
+    if (x_seq) { CK(cudaMemcpyAsync(x_seq, j.xseq, B * N * 24, cudaMemcpyDeviceToHost, h->stream)); h->stats.d2h_bytes += (long long)(B * N * 24); }
+    if (dt_out) { CK(cudaMemcpyAsync(dt_out, j.dt, B * 8, cudaMemcpyDeviceToHost, h->stream)); h->stats.d2h_bytes += (long long)(B * 8); }
+    if (status) { CK(cudaMemcpyAsync(status, j.status, B * 4, cudaMemcpyDeviceToHost, h->stream)); h->stats.d2h_bytes += (long long)(B * 4); }
+    if (kkt_err) { CK(cudaMemcpyAsync(kkt_err, j.kkt, B * 8, cudaMemcpyDeviceToHost, h->stream)); h->stats.d2h_bytes += (long long)(B * 8); }
+    if (iters) { CK(cudaMemcpyAsync(iters, j.iters, B * 4, cudaMemcpyDeviceToHost, h->stream)); h->stats.d2h_bytes += (long long)(B * 4); }
     CK(cudaStreamSynchronize(h->stream));
     return 0;
 }
 
 // ---- queue solve: `total` cold instances through the persistent kernel (continuous batching) ----------------------
-static int stream_reserve(mpcb200_handle* h, size_t total)
-{
-    if (total <= h->stream_cap) return 0;
-    void* old[] = {h->s_x0, h->s_xf, h->s_uprev, h->s_obst, h->s_vp, h->s_useq, h->s_xseq, h->s_dt, h->s_kkt, h->s_upacked, h->s_obst_count,
-                   h->s_obst_type, h->s_vp_count, h->s_status, h->s_iters};
-    for (void* p : old) if (p) cudaFree(p);
-    h->stream_cap = 0; h->s_obst_m = 0;
-    const size_t N = (size_t)h->n_cap, T = total;  // sized for the largest horizon the handle can be resampled to
-    CK(cudaMalloc(&h->s_x0, T * 3 * 8)); CK(cudaMalloc(&h->s_xf, T * 3 * 8)); CK(cudaMalloc(&h->s_uprev, T * 2 * 8));
-    CK(cudaMalloc(&h->s_obst, T * MAX_OBST * MPCB200_OBST_STRIDE * 8)); CK(cudaMalloc(&h->s_obst_count, T * 4)); CK(cudaMalloc(&h->s_obst_type, T * MAX_OBST * 4));
-    h->s_obst_m = MAX_OBST;
-    CK(cudaMalloc(&h->s_vp, T * MAX_VP * 3 * 8)); CK(cudaMalloc(&h->s_vp_count, T * 4));
-    CK(cudaMalloc(&h->s_useq, T * N * 2 * 8)); CK(cudaMalloc(&h->s_xseq, T * N * 3 * 8)); CK(cudaMalloc(&h->s_dt, T * 8)); CK(cudaMalloc(&h->s_kkt, T * 8));
-    CK(cudaMalloc(&h->s_upacked, T * (N - 1) * 2 * 8)); CK(cudaMalloc(&h->s_status, T * 4)); CK(cudaMalloc(&h->s_iters, T * 4));
-    h->stream_cap = total;
-    return 0;
-}
-
 extern "C" int mpcb200_solve_stream(mpcb200_handle* h, int total, const double* x0, const double* xf, const double* u_prev, double u_prev_dt,
                                     const mpcb200_obstacles* obst, const mpcb200_viapoints* vp, double* u_seq, double* x_seq, double* dt_out,
                                     int* status, double* kkt_err, int* iters, double* solve_time_s)
@@ -985,31 +975,10 @@ extern "C" int mpcb200_solve_stream(mpcb200_handle* h, int total, const double* 
     if (!h) return MPCB200_E_INVALID;
     if (total < 1 || !x0 || !xf) return set_err(h, MPCB200_E_INVALID, "total >= 1, x0 and xf are required");
     CK(cudaSetDevice(h->device));
-    int rc = stream_reserve(h, (size_t)total);
+    int rc = upload(h, h->queue, (size_t)total, x0, xf, u_prev, u_prev_dt, obst, vp, nullptr, nullptr);
     if (rc) return rc;
-    if ((rc = reserve_obstacles(h, true, h->stream_cap, (obst && obst->count) ? obst->max_per_instance : 0))) return rc;
-    const size_t T = (size_t)total, N = (size_t)h->cfg.n;
-    InputPtrs in;
-    Staging s{h->s_x0, h->s_xf, h->s_uprev, h->s_obst, h->s_vp, nullptr, h->s_obst_count, h->s_obst_type, h->s_vp_count, nullptr};
-    if ((rc = copy_inputs(h, s, T, x0, xf, u_prev, u_prev_dt, obst, vp, nullptr, nullptr, &in))) return rc;
-    OutputPtrs o{h->s_useq, h->s_xseq, h->s_dt, h->s_status, h->s_kkt, h->s_iters, h->s_upacked};
-    CK(cudaEventRecord(h->t0, h->stream));
-    if ((rc = launch_fused(h, total, 1, 1, in, o))) return rc;
-    CK(cudaEventRecord(h->t1, h->stream));
-    CK(cudaStreamSynchronize(h->stream));
-    float ms = 0.f;
-    CK(cudaEventElapsedTime(&ms, h->t0, h->t1));
-    if (solve_time_s) *solve_time_s = ms * 1e-3;
-    if ((rc = collect_fused_counters(h))) return rc;
-    // ---- results of the whole job ----
-    if (u_seq) { CK(cudaMemcpyAsync(u_seq, h->s_useq, T * N * 16, cudaMemcpyDeviceToHost, h->stream)); h->stats.d2h_bytes += (long long)(T * N * 16); }
-    if (x_seq) { CK(cudaMemcpyAsync(x_seq, h->s_xseq, T * N * 24, cudaMemcpyDeviceToHost, h->stream)); h->stats.d2h_bytes += (long long)(T * N * 24); }
-    if (dt_out) { CK(cudaMemcpyAsync(dt_out, h->s_dt, T * 8, cudaMemcpyDeviceToHost, h->stream)); h->stats.d2h_bytes += (long long)(T * 8); }
-    if (status) { CK(cudaMemcpyAsync(status, h->s_status, T * 4, cudaMemcpyDeviceToHost, h->stream)); h->stats.d2h_bytes += (long long)(T * 4); }
-    if (kkt_err) { CK(cudaMemcpyAsync(kkt_err, h->s_kkt, T * 8, cudaMemcpyDeviceToHost, h->stream)); h->stats.d2h_bytes += (long long)(T * 8); }
-    if (iters) { CK(cudaMemcpyAsync(iters, h->s_iters, T * 4, cudaMemcpyDeviceToHost, h->stream)); h->stats.d2h_bytes += (long long)(T * 4); }
-    CK(cudaStreamSynchronize(h->stream));
-    return 0;
+    if ((rc = solve_device(h, h->queue, 1, solve_time_s))) return rc;
+    return fetch(h, h->queue, u_seq, x_seq, dt_out, status, kkt_err, iters);
 }
 
 extern "C" int mpcb200_step_batch(mpcb200_handle* h, int B, const double* x0, const double* xf, const double* u_prev, double u_prev_dt,
@@ -1020,21 +989,11 @@ extern "C" int mpcb200_step_batch(mpcb200_handle* h, int B, const double* x0, co
     int rc = check_batch(h, B);
     if (rc) return rc;
     CK(cudaSetDevice(h->device));
-    if (h->solve_mode == 1)
-    {
-        if ((rc = upload_inputs(h, B, x0, xf, u_prev, u_prev_dt, obst, vp, x_init, reinit))) return rc;
-    }
-    else
-    {
-        // fused mode: the solve kernel reads the compact arrays itself, the blocks only carry the warm state
-        InputPtrs in;
-        if (!u_prev) CK(cudaMemsetAsync(h->d_uprev, 0, (size_t)B * 2 * 8, h->stream));
-        if ((rc = reserve_obstacles(h, false, (size_t)h->max_batch, (obst && obst->count) ? obst->max_per_instance : 0))) return rc;
-        if ((rc = copy_inputs(h, batch_staging(h), (size_t)B, x0, xf, u_prev, u_prev_dt, obst, vp, x_init, reinit, &in))) return rc;
-        h->B = B;
-    }
-    if ((rc = solve_device(h, B, 0, solve_time_s))) return rc;
-    return fetch_results(h, B, u_seq, x_seq, dt_out, status, kkt_err, iters);
+    if ((rc = upload(h, h->batch, (size_t)B, x0, xf, u_prev, u_prev_dt, obst, vp, x_init, reinit))) return rc;
+    // the phase kernels read the inputs from the instance blocks; the fused kernel reads the compact arrays itself
+    if (h->solve_mode == 1 && (rc = scatter_batch(h))) return rc;
+    if ((rc = solve_device(h, h->batch, 0, solve_time_s))) return rc;
+    return fetch(h, h->batch, u_seq, x_seq, dt_out, status, kkt_err, iters);
 }
 
 extern "C" int mpcb200_upload_inputs(mpcb200_handle* h, int B, const double* x0, const double* xf, const double* u_prev, double u_prev_dt,
@@ -1042,30 +1001,31 @@ extern "C" int mpcb200_upload_inputs(mpcb200_handle* h, int B, const double* x0,
 {
     int rc = check_batch(h, B);
     if (rc) return rc;
-    if ((rc = upload_inputs(h, B, x0, xf, u_prev, u_prev_dt, obst, vp, x_init, nullptr))) return rc;
+    CK(cudaSetDevice(h->device));
+    if ((rc = upload(h, h->batch, (size_t)B, x0, xf, u_prev, u_prev_dt, obst, vp, x_init, nullptr)) || (rc = scatter_batch(h))) return rc;
     CK(cudaStreamSynchronize(h->stream));
     return 0;
 }
 
 extern "C" int mpcb200_solve_resident(mpcb200_handle* h, int cold, double* solve_time_s)
 {
-    if (!h || h->B < 1) return set_err(h, MPCB200_E_INVALID, "no resident inputs: call mpcb200_upload_inputs first");
+    if (!h || h->batch.B < 1) return set_err(h, MPCB200_E_INVALID, "no resident inputs: call mpcb200_upload_inputs first");
     CK(cudaSetDevice(h->device));
-    return solve_device(h, h->B, cold ? 1 : 0, solve_time_s);
+    return solve_device(h, h->batch, cold ? 1 : 0, solve_time_s);
 }
 
 extern "C" int mpcb200_fetch_results(mpcb200_handle* h, double* u_seq, double* x_seq, double* dt_out, int* status, double* kkt_err, int* iters)
 {
-    if (!h || h->B < 1) return set_err(h, MPCB200_E_INVALID, "nothing to fetch");
+    if (!h || h->batch.B < 1) return set_err(h, MPCB200_E_INVALID, "nothing to fetch");
     CK(cudaSetDevice(h->device));
-    return fetch_results(h, h->B, u_seq, x_seq, dt_out, status, kkt_err, iters);
+    return fetch(h, h->batch, u_seq, x_seq, dt_out, status, kkt_err, iters);
 }
 
 extern "C" int mpcb200_device_controls(mpcb200_handle* h, void** dev_ptr, long long* n_doubles)
 {
-    if (!h || h->B < 1) return set_err(h, MPCB200_E_INVALID, "no batch solved yet");
-    if (dev_ptr) *dev_ptr = h->d_upacked;
-    if (n_doubles) *n_doubles = (long long)h->B * (h->cfg.n - 1) * 2;
+    if (!h || h->batch.B < 1) return set_err(h, MPCB200_E_INVALID, "no batch solved yet");
+    if (dev_ptr) *dev_ptr = h->batch.upacked;
+    if (n_doubles) *n_doubles = (long long)h->batch.B * (h->cfg.n - 1) * 2;
     return 0;
 }
 
@@ -1075,8 +1035,8 @@ extern "C" int mpcb200_reset(mpcb200_handle* h, const unsigned char* which, int 
     CK(cudaSetDevice(h->device));
     const int n = which ? B : h->max_batch;
     if (n < 1 || n > h->max_batch) return set_err(h, MPCB200_E_INVALID, "batch size out of range");
-    if (which) CK(cudaMemcpyAsync(h->d_reinit, which, (size_t)n, cudaMemcpyHostToDevice, h->stream));
-    reset_kernel<<<(n + 127) / 128, 128, 0, h->stream>>>(h->L, h->ws, n, which ? h->d_reinit : nullptr);
+    if (which) CK(cudaMemcpyAsync(h->batch.reinit, which, (size_t)n, cudaMemcpyHostToDevice, h->stream));
+    reset_kernel<<<(n + 127) / 128, 128, 0, h->stream>>>(h->L, h->ws, n, which ? h->batch.reinit.v : nullptr);
     CK(cudaGetLastError());
     CK(cudaStreamSynchronize(h->stream));
     return 0;
@@ -1090,7 +1050,8 @@ extern "C" int mpcb200_resample(mpcb200_handle* h, int n_new)
     CK(cudaSetDevice(h->device));
     const int B = h->max_batch, n_old = h->cfg.n;
     const int rec_words = MPCB200_SCAL_WORDS + 5 * h->n_cap;
-    if (!h->d_resample) CK(cudaMalloc(&h->d_resample, (size_t)B * rec_words * sizeof(double)));
+    const int rc = grow(h, h->d_resample, h->resample_cap, (size_t)B * rec_words * sizeof(double));
+    if (rc) return rc;
     resample_pack_kernel<<<(B + 127) / 128, 128, 0, h->stream>>>(h->L, h->ws, h->d_resample, rec_words, B);
     CK(cudaGetLastError());
     h->cfg.n = n_new;
@@ -1282,9 +1243,9 @@ extern "C" int mpcb200_stats_reset(mpcb200_handle* h)
 }
 extern "C" int mpcb200_export_controls(mpcb200_handle* h, void* dst_dev)
 {
-    if (!h || h->B < 1 || !dst_dev) return set_err(h, MPCB200_E_INVALID, "nothing to export");
+    if (!h || h->batch.B < 1 || !dst_dev) return set_err(h, MPCB200_E_INVALID, "nothing to export");
     CK(cudaSetDevice(h->device));
-    CK(cudaMemcpyAsync(dst_dev, h->d_upacked, (size_t)h->B * (h->cfg.n - 1) * 16, cudaMemcpyDeviceToDevice, h->stream));
+    CK(cudaMemcpyAsync(dst_dev, h->batch.upacked, (size_t)h->batch.B * (h->cfg.n - 1) * 16, cudaMemcpyDeviceToDevice, h->stream));
     CK(cudaStreamSynchronize(h->stream));
     return 0;
 }
@@ -1304,16 +1265,10 @@ static int costmap_run(mpcb200_handle* h, int B, const mpcb200_costmaps* maps, c
     const size_t mask_words = (size_t)B * nrb * Wp;
     const size_t need = (size_t)B * W * H + 16 + (size_t)B * 5 * 8 + 2 * (size_t)B * 4 + (size_t)B * M * (MPCB200_OBST_STRIDE * 8 + 4) +
                         mask_words * 4 + 512;
-    if (need > h->cm_cap)
-    {
-        CK(cudaStreamSynchronize(h->stream));
-        if (h->d_cm) cudaFree(h->d_cm);
-        h->d_cm = nullptr; h->cm_cap = 0;
-        CK(cudaMalloc(&h->d_cm, need));
-        h->cm_cap = need;
-    }
+    const int rc = grow(h, h->d_cm, h->cm_cap, need);
+    if (rc) return rc;
     // carve the scratch: 16-byte aligned pieces first (mask rows are stored as uint4), then ints, then the maps
-    char* p = (char*)h->d_cm;
+    char* p = h->d_cm;
     unsigned* d_mask = (unsigned*)p; p += mask_words * 4;
     double* s_params = (double*)p; p += (size_t)B * M * MPCB200_OBST_STRIDE * 8;
     double* d_origin = (double*)p; p += (size_t)B * 2 * 8;
@@ -1381,25 +1336,17 @@ extern "C" int mpcb200_step_batch_costmap(mpcb200_handle* h, int B, const double
     if (rc) return rc;
     if (max_per_instance < 1 || max_per_instance > MAX_OBST_LIST) return set_err(h, MPCB200_E_UNSUPPORTED, "step_batch_costmap: 1..2048 obstacles per instance");
     CK(cudaSetDevice(h->device));
+    Job& j = h->batch;
     // room for the lists in the batch's obstacle arrays
-    if ((rc = reserve_obstacles(h, false, (size_t)h->max_batch, max_per_instance))) return rc;
-    InputPtrs in;
-    if (!u_prev) CK(cudaMemsetAsync(h->d_uprev, 0, (size_t)B * 2 * 8, h->stream));
-    if ((rc = copy_inputs(h, batch_staging(h), (size_t)B, x0, xf, u_prev, u_prev_dt, nullptr, vp, x_init, reinit, &in))) return rc;
+    if ((rc = reserve(h, j, (size_t)B, max_per_instance))) return rc;
+    if ((rc = upload(h, j, (size_t)B, x0, xf, u_prev, u_prev_dt, nullptr, vp, x_init, reinit))) return rc;
     CostmapOut o;
-    if ((rc = costmap_run(h, B, maps, nullptr, h->d_x0, behind_robot_dist, max_per_instance, h->d_obst_count, h->d_obst_type, h->d_obst, &o))) return rc;
-    h->has_obst = 1; h->obst_max = max_per_instance;   // point obstacles only: no line-obstacle kernel variant needed
-    h->B = B;
-    if (h->solve_mode == 1)
-    {
-        in = batch_inputs(h, true);
-        scatter_inputs_kernel<<<grid_for(B, WARPS_PER_CTA), WARPS_PER_CTA * 32, 0, h->stream>>>(h->L, h->ws, B, in);
-        h->stats.launches_total += 1;
-        CK(cudaGetLastError());
-    }
-    if ((rc = solve_device(h, B, 0, solve_time_s))) return rc;
+    if ((rc = costmap_run(h, B, maps, nullptr, j.x0, behind_robot_dist, max_per_instance, j.obst_count, j.obst_type, j.obst, &o))) return rc;
+    j.obst_max = max_per_instance;   // point obstacles only: no line-obstacle kernel variant needed
+    if (h->solve_mode == 1 && (rc = scatter_batch(h))) return rc;
+    if ((rc = solve_device(h, j, 0, solve_time_s))) return rc;
     if (obst_found) CK(cudaMemcpyAsync(obst_found, o.found, (size_t)B * 4, cudaMemcpyDeviceToHost, h->stream));
-    rc = fetch_results(h, B, u_seq, x_seq, dt_out, status, kkt_err, iters);
+    rc = fetch(h, j, u_seq, x_seq, dt_out, status, kkt_err, iters);
     float ms = 0.f;
     if (!rc && cudaEventElapsedTime(&ms, h->c0, h->c1) == cudaSuccess) h->costmap_ms = ms;
     return rc;
@@ -1417,18 +1364,13 @@ extern "C" int mpcb200_check_feasible(mpcb200_handle* h, int B, const mpcb200_co
     if (!(inscribed_radius > 0) || !(min_resolution_angular > 0)) return set_err(h, MPCB200_E_INVALID, "check_feasible: inscribed_radius and min_resolution_angular must be > 0");
     const int n = x_seq ? n_poses : h->cfg.n;
     if (n < 1) return set_err(h, MPCB200_E_INVALID, "check_feasible: n_poses >= 1 required");
-    if (!x_seq && (h->B < B)) return set_err(h, MPCB200_E_INVALID, "check_feasible: no solved batch of this size on the device (pass x_seq)");
+    if (!x_seq && (h->batch.B < B)) return set_err(h, MPCB200_E_INVALID, "check_feasible: no solved batch of this size on the device (pass x_seq)");
     CK(cudaSetDevice(h->device));
     const size_t W = (size_t)maps->size_x, H = (size_t)maps->size_y;
     const size_t need = (size_t)B * n * 24 + (size_t)B * 16 + (size_t)(n_footprint > 0 ? n_footprint : 1) * 16 + (size_t)B * W * H + (size_t)B + 256;
-    if (need > h->fz_cap)
-    {
-        if (h->d_fz) cudaFree(h->d_fz);
-        h->d_fz = nullptr; h->fz_cap = 0;
-        CK(cudaMalloc(&h->d_fz, need));
-        h->fz_cap = need;
-    }
-    char* p = (char*)h->d_fz;
+    const int rc = grow(h, h->d_fz, h->fz_cap, need);
+    if (rc) return rc;
+    char* p = h->d_fz;
     double* d_x = (double*)p; p += (size_t)B * n * 24;
     double* d_origin = (double*)p; p += (size_t)B * 16;
     double* d_fp = (double*)p; p += (size_t)(n_footprint > 0 ? n_footprint : 1) * 16;
@@ -1439,7 +1381,7 @@ extern "C" int mpcb200_check_feasible(mpcb200_handle* h, int B, const mpcb200_co
     if (n_footprint > 0) CK(cudaMemcpyAsync(d_fp, footprint_xy, (size_t)n_footprint * 16, cudaMemcpyHostToDevice, h->stream));
     if (x_seq) CK(cudaMemcpyAsync(d_x, x_seq, (size_t)B * n * 24, cudaMemcpyHostToDevice, h->stream));
     h->stats.h2d_bytes += (long long)((size_t)B * W * H + (size_t)B * 16 + (size_t)n_footprint * 16 + (x_seq ? (size_t)B * n * 24 : 0));
-    FeasArgs a{maps->size_x, maps->size_y, maps->resolution, d_cost, d_origin, x_seq ? d_x : h->d_xseq, n, d_fp, n_footprint,
+    FeasArgs a{maps->size_x, maps->size_y, maps->resolution, d_cost, d_origin, x_seq ? d_x : h->batch.xseq.v, n, d_fp, n_footprint,
                inscribed_radius, min_resolution_angular, look_ahead_idx};
     feasible_kernel<<<grid_for(B, WARPS_PER_CTA), WARPS_PER_CTA * 32, 0, h->stream>>>(a, B, d_ok);
     h->stats.launches_total += 1;
@@ -1489,7 +1431,7 @@ struct mpcb200_multi
     std::vector<int> devices;
     std::vector<mpcb200_handle*> h;
     std::vector<void*> comm;
-    std::vector<double*> d_all;      // per device: gathered packed controls [n_dev][max_per][N-1][2]
+    std::vector<Dev<double>> d_all;  // per device: gathered packed controls [n_dev][max_per][N-1][2]
     NcclApi nccl;
     std::string err;
 };
@@ -1512,7 +1454,7 @@ extern "C" void mpcb200_destroy_multi(mpcb200_multi* m)
 {
     if (!m) return;
     for (size_t r = 0; r < m->comm.size(); ++r) if (m->comm[r] && m->nccl.CommDestroy) m->nccl.CommDestroy(m->comm[r]);
-    for (size_t r = 0; r < m->d_all.size(); ++r) if (m->d_all[r]) { cudaSetDevice(m->devices[r]); cudaFree(m->d_all[r]); }
+    for (size_t r = 0; r < m->d_all.size(); ++r) { cudaSetDevice(m->devices[r]); m->d_all[r].reset(); }
     for (auto* h : m->h) if (h) mpcb200_destroy(h);
     delete m;
 }
@@ -1524,7 +1466,7 @@ extern "C" int mpcb200_create_multi(const mpcb200_config* cfg, int max_batch_tot
     m->n_dev = n_devices; m->n = cfg->n;
     m->max_per = (max_batch_total + n_devices - 1) / n_devices;
     m->devices.assign(devices, devices + n_devices);
-    m->h.assign(n_devices, nullptr); m->comm.assign(n_devices, nullptr); m->d_all.assign(n_devices, nullptr);
+    m->h.assign(n_devices, nullptr); m->comm.assign(n_devices, nullptr); m->d_all = std::vector<Dev<double>>(n_devices);
     for (int r = 0; r < n_devices; ++r)
     {
         const int rc = mpcb200_create(cfg, m->max_per, devices[r], &m->h[r]);
@@ -1540,7 +1482,7 @@ extern "C" int mpcb200_create_multi(const mpcb200_config* cfg, int max_batch_tot
     const size_t words = (size_t)n_devices * m->max_per * (cfg->n - 1) * 2;
     for (int r = 0; r < n_devices; ++r)
     {
-        if (cudaSetDevice(devices[r]) != cudaSuccess || cudaMalloc(&m->d_all[r], words * 8) != cudaSuccess)
+        if (cudaSetDevice(devices[r]) != cudaSuccess || alloc(m->d_all[r], words) != cudaSuccess)
         { mpcb200_destroy_multi(m); return multi_err(nullptr, MPCB200_E_CUDA, "cudaMalloc of the gathered controls failed"); }
     }
     *out = m;
@@ -1613,7 +1555,7 @@ extern "C" int mpcb200_step_batch_multi(mpcb200_multi* m, int B, const double* x
         for (int r = 0; r < G && nrc == 0; ++r)
         {
             cudaSetDevice(m->devices[r]);
-            nrc = m->nccl.AllGather(m->h[r]->d_upacked, m->d_all[r], count, MPC_NCCL_FLOAT64, m->comm[r], m->h[r]->stream);
+            nrc = m->nccl.AllGather(m->h[r]->batch.upacked, m->d_all[r], count, MPC_NCCL_FLOAT64, m->comm[r], m->h[r]->stream);
         }
         const int erc = m->nccl.GroupEnd();
         if (nrc == 0) nrc = erc;
@@ -1627,7 +1569,7 @@ extern "C" int mpcb200_step_batch_multi(mpcb200_multi* m, int B, const double* x
     else
     {
         cudaSetDevice(m->devices[0]);
-        if (cudaMemcpyAsync(m->d_all[0], m->h[0]->d_upacked, count * 8, cudaMemcpyDeviceToDevice, m->h[0]->stream) != cudaSuccess ||
+        if (cudaMemcpyAsync(m->d_all[0], m->h[0]->batch.upacked, count * 8, cudaMemcpyDeviceToDevice, m->h[0]->stream) != cudaSuccess ||
             cudaStreamSynchronize(m->h[0]->stream) != cudaSuccess)
             return multi_err(m, MPCB200_E_CUDA, "copy of the controls failed");
     }
